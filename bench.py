@@ -4,6 +4,7 @@
 
   python bench.py --gpus 1 --steps 20 --warmup 3            # our arm (sm_100a engine)
   python bench.py --impl reference --steps 2 --warmup 1     # reference arm: the reference path on the host cores
+  python bench.py --steps 20 --dump-outputs DIR            # also write the outputs of the last timed step as DIR/<name>.npy
 
 A "step" = one pass of the whole hot path (trunk, FPN, RPN, proposals, RoIAlign, box head, per-class NMS,
 mask head) over one batch of synthetic images.  `value` is timed with inputs resident in HBM (CUDA-graph replay of
@@ -245,6 +246,28 @@ def microbench_roialign(torch, dev, hbm_peak, which):
     return roof, rows
 
 
+def dump_outputs(out_dir, eng):
+    """Writes what the last timed step computed, the arrays detector.detect() returns for that batch (boxes, scores, classes, counts,
+    roi_idx, masks of the detected class, range_flag), to out_dir/<name>.npy as float32 (float64 for the integer arrays): about 3 MB at
+    batch 8.  Slots past an image's detection count hold no result and are written as zeros, so that the outputs of two builds on the
+    same (seeded) inputs can be compared array for array."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    counts = eng.buffer("det_counts").cpu().numpy().astype(np.int64)
+    B = len(counts)
+    arrays = {"boxes": eng.buffer("det_boxes"), "scores": eng.buffer("det_scores"), "classes": eng.buffer("det_classes"),
+              "roi_idx": eng.buffer("det_roi_idx"), "masks": eng.buffer("masks")}
+    for name, t in arrays.items():
+        a = t.cpu().numpy()
+        a = a.reshape((B, -1) + a.shape[1:] if name == "masks" else a.shape)          # masks: [B * cap, 28, 28] -> [B, cap, 28, 28]
+        a = a.astype(np.float32 if a.dtype.kind == "f" else np.float64)
+        for b in range(B):
+            a[b, counts[b]:] = 0
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    np.save(os.path.join(out_dir, "counts.npy"), counts.astype(np.float64))
+    np.save(os.path.join(out_dir, "range_flag.npy"), eng.buffer("range_flag").cpu().numpy().astype(np.float64))
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -323,6 +346,8 @@ def run_ours(args):
     eng.check_range()      # the kind::f16 conv path raises a device flag if an activation left the fp16 range (never on this workload)
     rois_per_image = float(eng.buffer("roi_counts").float().mean().item())
     dets_per_image = float(eng.buffer("det_counts").float().mean().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng)         # the engine buffers still hold the last timed step (batch (steps - 1) % 2)
 
     # ---- (B) end to end through the public call with HOST buffers: model.detect(pinned host batch) uploads through its two staging
     # buffers on a copy stream (H2D of step i+1 overlaps the compute of step i); every step's results are read back to pinned host memory
@@ -481,7 +506,10 @@ def main():
     ap.add_argument("--no-config1", action="store_true", help="reference arm: skip the Fast R-CNN R-50-C4 (configs[0]) CPU timing")
     ap.add_argument("--arch", default="resnet50", choices=["resnet50", "resnet101"],
                     help="resnet101 = BASELINE.json configs[3] model (not the headline metric)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

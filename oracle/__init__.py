@@ -1,6 +1,11 @@
 """ORACLE -- test infrastructure only (never imported by detectorch_b200/)."""
 import os
 
+# torch-CPU results depend, in the last bits, on the instruction set ATen / oneDNN / MKL pick and on the thread count.  The bit-exact
+# fixture of the reference detector's outputs (tests/golden/net_golden_r50fpn_128x160.npz) is produced and checked under this
+# environment (AVX2 code paths, one thread), so that it holds on any x86-64 host with AVX2.  It must be set before torch starts.
+CPU_BITWISE_ENV = {"ATEN_CPU_CAPABILITY": "avx2", "ONEDNN_MAX_CPU_ISA": "AVX2", "MKL_CBWR": "AVX2", "OMP_NUM_THREADS": "1", "MKL_NUM_THREADS": "1"}
+
 
 def usable_cpus():
     """Host threads this process may really use: the scheduler affinity mask, capped by the cgroup CPU quota (cpu.max) when there is one.

@@ -6,6 +6,7 @@ fixtures are committed so the GPU box (which has no reference tree) can pin agai
     python tests/golden/make_golden.py
 """
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -13,6 +14,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
+from oracle import CPU_BITWISE_ENV  # noqa: E402
 from oracle import reference_shim as rs  # noqa: E402
 from oracle import network as net  # noqa: E402
 from oracle import ref as oref  # noqa: E402
@@ -106,9 +108,22 @@ def main():
     G["pp_mask_restore"] = bm['rois_idx_restore_int32']
     for l in range(2, 6):
         G["pp_mask_rois_fpn%d" % l] = bm['rois_fpn%d' % l]
-    np.savez_compressed(os.path.join(OUT, "ops_golden.npz"), **G)
+    # the RoIAlign forward vectors go to a file of their own so that each fixture stays under 1 MB
+    np.savez_compressed(os.path.join(OUT, "roialign_golden.npz"), **{k: v for k, v in G.items() if k.startswith("roi_")})
+    np.savez_compressed(os.path.join(OUT, "ops_golden.npz"), **{k: v for k, v in G.items() if not k.startswith("roi_")})
+    # the detector fixture is bit-exact only under the pinned torch-CPU configuration that tests/test_oracle.py checks it with
+    subprocess.check_call([sys.executable, os.path.abspath(__file__), "--detector"], env=dict(os.environ, **CPU_BITWISE_ENV))
+    for f in ("ops_golden.npz", "roialign_golden.npz", "net_golden_r50fpn_128x160.npz"):
+        print(f, os.path.getsize(os.path.join(OUT, f)) // 1024, "KiB")
 
-    # ---- the reference detector end to end (tiny image, synthetic weights shared by name)
+
+def detector_golden():
+    """The reference detector end to end (tiny image, synthetic weights shared by name)."""
+    rs.install()
+    import utils.result_utils as ru
+    from utils.multilevel_rois import add_multilevel_rois_for_test
+    from model.detector import detector
+    torch.set_num_threads(1)
     m = detector(arch='resnet50', conv_body_layers=['conv1', 'bn1', 'relu', 'maxpool', 'layer1', 'layer2', 'layer3', 'layer4'],
                  conv_head_layers='two_layer_mlp', fpn_layers=['layer1', 'layer2', 'layer3', 'layer4'], fpn_extra_lvl=True,
                  roi_height=7, roi_width=7, roi_spatial_scale=[0.25, 0.125, 0.0625, 0.03125], roi_sampling_ratio=2,
@@ -134,9 +149,7 @@ def main():
     N["det_classes"] = cls_of_det.astype(np.int64)
     N["masks_own_class"] = masks.numpy()[np.arange(len(cls_of_det)), cls_of_det][:, ::2, ::2].copy()
     np.savez_compressed(os.path.join(OUT, "net_golden_r50fpn_128x160.npz"), **N)
-    for f in ("ops_golden.npz", "net_golden_r50fpn_128x160.npz"):
-        print(f, os.path.getsize(os.path.join(OUT, f)) // 1024, "KiB")
 
 
 if __name__ == "__main__":
-    main()
+    detector_golden() if "--detector" in sys.argv else main()

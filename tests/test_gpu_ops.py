@@ -19,7 +19,9 @@ def dev(built):
 
 @pytest.fixture(scope="module")
 def G():
-    return np.load(os.path.join(GOLD, "ops_golden.npz"))
+    g = dict(np.load(os.path.join(GOLD, "ops_golden.npz")))
+    g.update(np.load(os.path.join(GOLD, "roialign_golden.npz")))
+    return g
 
 
 def _boxes(rng, n, W=1216, H=800):

@@ -1,8 +1,10 @@
 """CPU test of the Detectron caffe2-pickle weight import (SURVEY.md 8f "next" row 2): a synthetic pickle written with the
-reference's own blob names loads identically into the reference detector and into the detectorch_b200 mirror, for the
+reference's own blob names loads into the detectorch_b200 mirror exactly as it loads into the reference detector, for the
 constructor kwargs of every eval_*.ipynb notebook (Fast / Faster / Mask R-CNN on the C4 and on the FPN body: the loader
 branches on use_rpn_head / use_fpn_body / mask_head_type / two_layer_mlp exactly like detector.py:317-374).
-Needs the reference tree (its utils.utils.parse_th_to_caffe2 name mapping), so it is skipped on the GPU box."""
+The blob names (the reference's utils.utils.parse_th_to_caffe2) and what the reference's loader made of each pickle are stored in
+tests/golden/pickle_golden.npz (tests/golden/make_crosscheck_golden.py runs the reference to produce them)."""
+import hashlib
 import os
 import pickle
 
@@ -11,7 +13,6 @@ import pytest
 import torch
 
 from oracle import network as net
-from oracle import reference_shim as rs
 
 FPN = dict(arch='resnet50', conv_body_layers=['conv1', 'bn1', 'relu', 'maxpool', 'layer1', 'layer2', 'layer3', 'layer4'],
            conv_head_layers='two_layer_mlp', fpn_layers=['layer1', 'layer2', 'layer3', 'layer4'],
@@ -27,77 +28,51 @@ CONFIGS = {
 }
 
 
-def write_detectron_pickle(path, ref_model, P, flags):
-    """A pickle in the published checkpoints' format ({'blobs': {caffe2 name: ndarray}}), filled from the flat parameter dict P."""
-    from utils.utils import parse_th_to_caffe2
-    blobs = {}
-    for k in ref_model.model.state_dict().keys():                            # trunk: torchvision name -> caffe2 blob name
-        if 'running' in k or 'fc' in k:
-            continue
-        if 'num_batches' in k:
-            # torch >= 0.4.1 adds this buffer; the reference's loader (detector.py:300-304) does not skip it, so a blob must exist
-            blobs[parse_th_to_caffe2(k.split('.'))] = np.zeros((), np.float32)
-            continue
-        w = P["model." + k].numpy()
-        blobs[parse_th_to_caffe2(k.split('.'))] = w[:, (2, 1, 0), :, :].copy() if k == 'conv1.weight' else w     # pickles hold BGR
+GOLD = os.path.join(os.path.dirname(__file__), "golden", "pickle_golden.npz")
 
-    def put(wn, bn, name):
-        blobs[wn], blobs[bn] = P[name + ".weight"].numpy(), P[name + ".bias"].numpy()
-    put('bbox_pred_w', 'bbox_pred_b', 'bbox_head'); put('cls_score_w', 'cls_score_b', 'classif_head')
-    if flags["rpn"]:
-        sfx = '_fpn2' if flags["fpn"] else ''
-        put('conv_rpn%s_w' % sfx, 'conv_rpn%s_b' % sfx, 'rpn.conv_rpn')
-        put('rpn_cls_logits%s_w' % sfx, 'rpn_cls_logits%s_b' % sfx, 'rpn.rpn_cls_prob')
-        put('rpn_bbox_pred%s_w' % sfx, 'rpn_bbox_pred%s_b' % sfx, 'rpn.rpn_bbox_pred')
-    if flags["mask"]:
-        put('conv5_mask_w', 'conv5_mask_b', 'mask_head.transposed_conv'); put('mask_fcn_logits_w', 'mask_fcn_logits_b', 'mask_head.classif_logits')
-        if flags["fpn"]:
-            for i in range(1, 5):
-                put('_[mask]_fcn%d_w' % i, '_[mask]_fcn%d_b' % i, 'mask_head.conv_head.fcn%d' % i)
-    if flags["fpn"]:
-        for i, l in enumerate(FPN['fpn_layers']):
-            kc = parse_th_to_caffe2((l + '.' + list(getattr(ref_model.model, l).state_dict().keys())[-1]).split('.'))
-            kc = kc[:kc.rfind("_")]
-            suffix = '_sum_lateral' if i < 3 else '_sum'
-            put('fpn_inner_' + kc + suffix + '_w', 'fpn_inner_' + kc + suffix + '_b', 'conv_body.fpn_lateral.%d' % i)
-            put('fpn_' + kc + '_sum_w', 'fpn_' + kc + '_sum_b', 'conv_body.fpn_output.%d' % i)
-        put('fc6_w', 'fc6_b', 'conv_head.fc6'); put('fc7_w', 'fc7_b', 'conv_head.fc7')
+
+def sha1(t):
+    return hashlib.sha1(np.ascontiguousarray(t.detach().cpu().numpy()).tobytes()).hexdigest()
+
+
+def write_detectron_pickle(path, G, name, P):
+    """A pickle in the published checkpoints' format ({'blobs': {caffe2 name: ndarray}}), filled from the flat parameter dict P by the
+    recipe stored for this configuration (blob name, parameter it holds or '' for a zero blob, BGR stem flag)."""
+    blobs = {}
+    for blob, src, bgr in zip(G[name + "_blob"], G[name + "_src"], G[name + "_bgr"]):
+        w = P[str(src)].numpy() if src else np.zeros((), np.float32)
+        blobs[str(blob)] = w[:, (2, 1, 0), :, :].copy() if bgr else w     # pickles hold BGR
     with open(path, "wb") as f:
         pickle.dump({'blobs': blobs}, f, protocol=2)
 
 
-@pytest.mark.skipif(not rs.available(), reason="reference tree not present")
 @pytest.mark.parametrize("name", sorted(CONFIGS))
 def test_detectron_pickle_loads_like_the_reference(tmp_path, built, name):
-    rs.install()
-    from model.detector import detector as ref_detector                 # the reference
     from detectorch_b200.model.detector import detector as b200_detector
+    G = np.load(GOLD)
     kw, flags = CONFIGS[name]
     P = net.synthetic_params("resnet50", **flags)
-    ref_kw = dict(kw, roi_feature_channels=1024) if flags["fpn"] else kw   # the FPN notebooks rely on the pickle to resize the 2048-wide default heads
     pkl = os.path.join(str(tmp_path), "model_final.pkl")
-    write_detectron_pickle(pkl, ref_detector(**ref_kw), P, flags)
-    ref = ref_detector(detector_pkl_file=pkl, **kw)                     # exactly the notebook's cell 7
-    mine = b200_detector(detector_pkl_file=pkl, **kw)
-    sr, sm = ref.state_dict(), mine.state_dict()
-    for k, v in P.items():
-        assert torch.equal(sr[k], v), "reference loader: " + k           # the synthetic pickle round-trips through the reference
-        assert torch.equal(sm[k], v), "mirror loader: " + k
+    write_detectron_pickle(pkl, G, name, P)
+    mine = b200_detector(detector_pkl_file=pkl, **kw)                    # exactly the notebook's cell 7
+    sm = mine.state_dict()
+    assert [str(k) for k in G[name + "_keys"]] == sorted(P)
+    for k, want in zip(G[name + "_keys"], G[name + "_sha1"]):
+        k = str(k)
+        assert torch.equal(sm[k], P[k]), "mirror loader: " + k
+        assert sha1(sm[k]) == str(want), "differs from the reference loader: " + k
     # and the engine's parameter table accepts exactly these names
     from detectorch_b200 import engine
     t = engine.param_table("resnet50", use_mask=flags["mask"], model="fpn" if flags["fpn"] else "c4", use_rpn=flags["rpn"])
     assert set(t) == set(P) and all(t[k] == int(np.prod(P[k].shape)) for k in P)
 
 
-@pytest.mark.skipif(not rs.available(), reason="reference tree not present")
 def test_caffe2_blob_names_match_the_reference_helper():
     """The mirror's own torchvision-name -> caffe2-blob-name mapping equals utils/utils.py:44-71 (parse_th_to_caffe2) on every trunk key."""
-    rs.install()
-    import torchvision.models as models
-    from utils.utils import parse_th_to_caffe2
     from detectorch_b200.model.detector import caffe2_blob_name
+    G = np.load(GOLD)
     for arch in ("resnet50", "resnet101"):
-        keys = [k for k in getattr(models, arch)().state_dict().keys() if not ('running' in k or 'fc' in k or 'num_batches' in k)]
-        assert len(keys) > 150
-        for k in keys:
-            assert caffe2_blob_name(k) == parse_th_to_caffe2(k.split('.')), k
+        keys, names = G["names_%s_keys" % arch], G["names_%s_blobs" % arch]
+        assert len(keys) > 150 and len(keys) == len(names)
+        for k, n in zip(keys, names):
+            assert caffe2_blob_name(str(k)) == str(n), k
