@@ -503,24 +503,90 @@ __global__ void fp16_split_kernel(const float* __restrict__ w, float mult, __hal
     }
 }
 
+void fill_plan(const ConvLayer& L, int inst, int num_kb, dt_conv_plan* o) {
+    memset(o, 0, sizeof(*o));
+    o->instantiation = inst;
+    if (inst >= 0) {
+        const ConvInstance& r = kConvInstances[inst];
+        o->block_n = r.bn; o->nmain = r.nmain; o->two_sm = r.two_sm; o->kind = r.kind; o->ring = r.ring; o->slots = r.slots; o->halo = r.halo;
+        o->ws = r.ws;
+    }
+    const ConvParams& p = L.p;
+    o->wbox = p.wbox; o->hbox = p.hbox; o->nbox = p.nbox; o->tiles_w = p.tiles_w; o->tiles_h = p.tiles_h; o->tiles_n = p.tiles_n;
+    o->m_pairs = p.m_pairs; o->n_tiles = p.n_tiles; o->grid = (int)L.grid.x; o->num_kb = num_kb; o->ho = p.ho; o->wo = p.wo;
+}
+
+// plan (and, launch != 0, run) a built layer
+int plan_and_launch(const ConvLayer& L, int num_kb, dt_conv_plan* plan_out, int launch, dt_stream_t stream) {
+    const int inst = conv_instance_of(L);
+    if (plan_out) fill_plan(L, inst, num_kb, plan_out);
+    if (inst < 0) { fprintf(stderr, "[detectorch_b200] conv: no kernel instantiation for this layer\n"); return 0; }
+    if (launch) DT_CHECK_CUDA(kConvInstances[inst].launch(L, (cudaStream_t)stream));
+    return 1;
+}
+}  // namespace
+
+extern "C" int dt_conv2d_spec(const dt_conv_desc* d, dt_conv_plan* plan_out, int launch, dt_stream_t stream) {
+    if (!d) return 0;
+    ConvSpec s;
+    memset(&s, 0, sizeof(s));
+    s.kind = d->kind == 1 ? KIND_F16X3 : KIND_TF32X3;
+    s.x = reinterpret_cast<const float*>(d->x); s.x_lo = d->x_lo; s.N = d->N; s.H = d->H; s.W = d->W; s.Cin = d->Cin;
+    s.x_pix_stride = d->x_pix_stride > 0 ? d->x_pix_stride : d->Cin; s.x_mult = d->x_multiplier;
+    s.w_hi = d->w_hi; s.w_lo = d->w_lo; s.range_flag = d->range_flag;
+    s.Cout = d->Cout; s.kh = d->kh; s.kw = d->kw; s.pad = d->pad; s.stride = d->stride;
+    s.scale = d->scale; s.shift = d->shift;
+    s.y = reinterpret_cast<float*>(d->y); s.y_lo = d->y_lo; s.y_pix_stride = d->y_pix_stride > 0 ? d->y_pix_stride : d->Cout;
+    s.out_h = d->out_h; s.out_w = d->out_w; s.out_step = d->out_step; s.out_y0 = d->out_y0; s.out_x0 = d->out_x0;
+    s.residual = d->residual; s.res_pix_stride = d->res_pix_stride > 0 ? d->res_pix_stride : d->Cout;
+    s.up_src = d->up_src; s.up_h = d->up_h; s.up_w = d->up_w;
+    s.res_mode = d->res_mode; s.relu = d->relu; s.sigmoid_ch = d->sigmoid_ch; s.passes = d->passes;
+    s.tap0 = d->tap0; s.ntaps = d->ntaps; s.force_block_n = d->force_block_n; s.precise = d->precise; s.no_merge = d->no_merge;
+    ConvLayer L;
+    if (!conv_build(s, &L)) return 0;
+    const int num_kb = L.p.ntaps * L.p.cin_blocks;
+    return plan_and_launch(L, num_kb, plan_out, launch, stream);
+}
+
+extern "C" int dt_conv2d_stem(const void* x4, int planes, int B, int Hp, int Wp, int H1, int W1, const void* w_hi, const void* w_lo, int kind,
+                              const float* scale, const float* shift, float x_multiplier, int passes, int* range_flag, float* y,
+                              dt_conv_plan* plan_out, int launch, dt_stream_t stream) {
+    ConvLayer L;
+    if (!conv_build_stem(reinterpret_cast<const float*>(x4), B, Hp, Wp, H1, W1, w_hi, w_lo, scale, shift, y, passes, &L,
+                         kind == 1 ? KIND_F16X3 : KIND_TF32X3, range_flag, planes != 0, x_multiplier)) {
+        fprintf(stderr, "[detectorch_b200] dt_conv2d_stem: the layer could not be built\n");
+        return 0;
+    }
+    return plan_and_launch(L, 7, plan_out, launch, stream);
+}
+
+extern "C" int dt_conv_instantiation_count(void) { return kNumConvInstances; }
+
+extern "C" int dt_conv_instantiation_info(int i, int* fields8) {
+    if (i < 0 || i >= kNumConvInstances || !fields8) return 0;
+    const ConvInstance& r = kConvInstances[i];
+    const int f[8] = {r.bn, r.nmain, r.two_sm, r.kind, r.ring, r.slots, r.halo, r.ws};
+    memcpy(fields8, f, sizeof(f));
+    return 1;
+}
+
+namespace {
 int conv2d_nhwc_impl(int kind, const float* x, int N, int H, int W, int Cin, int x_pix_stride, const void* w, const void* w_lo, int Cout, int kh,
                      int kw, int pad, int stride, const float* scale, const float* shift, const float* residual, int res_mode,
                      const float* up_src, int up_h, int up_w, int relu, int sigmoid_ch, int passes, int force_block_n, int* range_flag,
                      float* y, int y_pix_stride, dt_stream_t stream) {
-    ConvSpec s;
-    memset(&s, 0, sizeof(s));
-    s.x = x; s.N = N; s.H = H; s.W = W; s.Cin = Cin; s.x_pix_stride = x_pix_stride;
-    s.w_hi = w; s.w_lo = w_lo; s.kind = kind; s.range_flag = range_flag;
-    s.Cout = Cout; s.kh = kh; s.kw = kw; s.pad = pad; s.stride = stride;
-    s.scale = scale; s.shift = shift; s.y = y; s.y_pix_stride = y_pix_stride;
-    s.residual = residual; s.res_pix_stride = Cout; s.up_src = up_src; s.up_h = up_h; s.up_w = up_w;
-    s.res_mode = res_mode; s.relu = relu; s.sigmoid_ch = sigmoid_ch; s.passes = passes; s.force_block_n = force_block_n;
-    s.precise = force_block_n < 0;
-    if (force_block_n < 0) s.force_block_n = 128;        // -1: the precise 128-wide tile (3 rotating accumulators)
-    ConvLayer L;
-    if (!conv_build(s, &L)) return 0;
-    DT_CHECK_CUDA(conv_launch(L, (cudaStream_t)stream));
-    return 1;
+    dt_conv_desc d;
+    memset(&d, 0, sizeof(d));
+    d.kind = kind == KIND_F16X3 ? 1 : 0;
+    d.x = x; d.N = N; d.H = H; d.W = W; d.Cin = Cin; d.x_pix_stride = x_pix_stride;
+    d.w_hi = w; d.w_lo = w_lo; d.range_flag = range_flag;
+    d.Cout = Cout; d.kh = kh; d.kw = kw; d.pad = pad; d.stride = stride;
+    d.scale = scale; d.shift = shift; d.y = y; d.y_pix_stride = y_pix_stride;
+    d.residual = residual; d.res_pix_stride = Cout; d.up_src = up_src; d.up_h = up_h; d.up_w = up_w;
+    d.res_mode = res_mode; d.relu = relu; d.sigmoid_ch = sigmoid_ch; d.passes = passes; d.force_block_n = force_block_n;
+    d.precise = force_block_n < 0;
+    if (force_block_n < 0) d.force_block_n = 128;        // -1: the precise 128-wide tile (3 rotating accumulators)
+    return dt_conv2d_spec(&d, nullptr, 1, stream);
 }
 }  // namespace
 

@@ -143,6 +143,8 @@ struct ConvSpec {
     int force_block_n;                            // 0 = auto
     int precise;                                  // BLOCK_N == 128 only: 3 rotating accumulators instead of TMEM double-buffering
     int no_merge;                                 // keep the cross terms in their own accumulator whatever K is (mask head: tightest parity bar)
+    float x_mult;                                 // KIND_F16X3, fp32 input: power of two applied to x before the fp16 split (0 or 1: none);
+                                                  // the caller folds 1 / x_mult into scale.  Keeps the low half of small activations normal.
 };
 
 inline void choose_box(int Wo, int Ho, int N, int max_w, int* wbox, int* hbox, int* nbox) {
@@ -249,6 +251,10 @@ inline bool conv_build(const ConvSpec& s, ConvLayer* L) {
         }
         if (best < 0) L->halo = 0; else wbox = 8;
     }
+    if (s.x_mult != 0.f && s.x_mult != 1.f && (s.kind != KIND_F16X3 || s.x_lo)) {
+        fprintf(stderr, "[detectorch_b200] conv_build: an input multiplier needs the f16 kind and an fp32 input\n");
+        return false;
+    }
     const int abox_w = L->halo ? wbox + 2 : wbox * s.stride;
     const int K = s.kh * s.kw * s.Cin;
     const uint64_t xs = (uint64_t)s.x_pix_stride * 4;
@@ -272,6 +278,7 @@ inline bool conv_build(const ConvSpec& s, ConvLayer* L) {
     }
     L->kind = s.kind == KIND_F16X3 ? KIND_F16X3 : KIND_TF32X3;
     p.range_flag = s.range_flag;
+    p.a_mult = (s.x_mult != 1.f) ? s.x_mult : 0.f;
     const uint64_t ys = (uint64_t)s.y_pix_stride * 4;
     if (s.y_lo) {
         if (s.kind != KIND_F16X3 || s.out_step != 0 || s.y_pix_stride != s.Cout || s.res_mode != RES_NONE || (s.Cout % 32) != 0) {
@@ -286,6 +293,11 @@ inline bool conv_build(const ConvSpec& s, ConvLayer* L) {
     } else if (s.out_step == 0) {
         if (!make_tmap_4d(&p.tm_d, s.y, s.Cout, Wo, Ho, s.N, ys, ys * Wo, ys * Wo * Ho, 32, wbox, hbox, nbox)) return false;
     } else {
+        if (s.out_step < 0 || s.out_y0 < 0 || s.out_x0 < 0 || (Ho - 1) * s.out_step + s.out_y0 >= s.out_h ||
+            (Wo - 1) * s.out_step + s.out_x0 >= s.out_w) {
+            fprintf(stderr, "[detectorch_b200] conv_build: the output remap scatters outside the [N,out_h,out_w] map\n");
+            return false;
+        }
         // strided scatter view: logical (w,h) -> physical (w*step + x0, h*step + y0) of an [N,out_h,out_w] map
         const float* base = s.y + ((size_t)s.out_y0 * s.out_w + s.out_x0) * s.y_pix_stride;
         if (!make_tmap_4d(&p.tm_d, base, s.Cout, Wo, Ho, s.N, ys * s.out_step, ys * s.out_w * s.out_step, ys * s.out_w * s.out_h, 32,
@@ -363,7 +375,7 @@ inline bool conv_build(const ConvSpec& s, ConvLayer* L) {
 // hit zero weights).  K = 7 x 32.  H uses elementStride 2.
 inline bool conv_build_stem(const float* x4, int B, int Hp, int Wp, int H1, int W1, const void* w_hi, const void* w_lo, const float* scale,
                             const float* shift, float* y, int passes, ConvLayer* L, int kind = KIND_TF32X3, int* range_flag = nullptr,
-                            bool x4_planes = false) {
+                            bool x4_planes = false, float x_mult = 0.f) {
     memset(&L->p, 0, sizeof(ConvParams));
     ConvParams& p = L->p;
     int wbox, hbox, nbox;
@@ -397,6 +409,10 @@ inline bool conv_build_stem(const float* x4, int B, int Hp, int Wp, int H1, int 
     }
     L->kind = kind == KIND_F16X3 ? KIND_F16X3 : KIND_TF32X3;
     p.range_flag = range_flag;
+    if (x_mult != 0.f && x_mult != 1.f) {
+        if (kind != KIND_F16X3 || x4_planes) return false;
+        p.a_mult = x_mult;
+    }
     const uint64_t ys = 64 * 4;
     if (!make_tmap_4d(&p.tm_d, y, 64, W1, H1, B, ys, ys * W1, ys * W1 * H1, 32, wbox, hbox, nbox)) return false;
     p.scale = scale; p.shift = shift;
@@ -449,57 +465,76 @@ inline cudaError_t conv_launch_cfg(const ConvLayer& L, cudaStream_t stream) {
     return cudaGetLastError();
 }
 
-template <bool TWO, int KIND>
-inline cudaError_t conv_launch_sm(const ConvLayer& L, cudaStream_t stream) {
-    // two staging slots only in the kind::f16 kernels (the engine default): the tf32 kind's stages are 64-96 KB
-    constexpr bool kCan2 = KIND == KIND_F16X3;
-    const bool s2 = kCan2 && L.slots == 2;
-    constexpr int S2 = kCan2 ? 2 : 1;
-    if constexpr (KIND == KIND_F16X3) {
-        if (L.halo) {
-            if constexpr (TWO) {
-                if (L.block_n == 128 && L.halo == 1) return conv_launch_cfg<128, 1, true, KIND_F16X3, 0, 2, 1>(L, stream);
-                if (L.block_n == 64 && L.halo == 1 && L.ws) return conv_launch_cfg<64, 3, true, KIND_F16X3, 0, 2, 1, true>(L, stream);
-                if (L.block_n == 64 && L.halo == 2 && L.ws)
-                    return L.nmain == 1 ? conv_launch_cfg<64, 1, true, KIND_F16X3, 0, 2, 2, true>(L, stream)
-                                        : conv_launch_cfg<64, 3, true, KIND_F16X3, 0, 2, 2, true>(L, stream);
-            } else {
-                if (L.block_n == 64 && L.halo == 1) return conv_launch_cfg<64, 3, false, KIND_F16X3, 0, 2, 1>(L, stream);
-                if (L.block_n == 64 && L.halo == 2) return conv_launch_cfg<64, 3, false, KIND_F16X3, 0, 2, 2>(L, stream);
-            }
-            return cudaErrorInvalidValue;
-        }
+// Every instantiation of conv_tcgen05_kernel, one row each.  conv_instance_of() maps a built layer to its row; the launcher and the
+// plan report (dt_conv2d_spec) both go through it, and dt_conv_instantiation_info exports the table.
+struct ConvInstance {
+    int bn, nmain, two_sm, kind, ring, slots, halo, ws;
+    cudaError_t (*launch)(const ConvLayer&, cudaStream_t);
+};
+#define DT_CONV_ROW(BN, NM, TWO, KIND, RING, SLOTS, HALO, WS) \
+    { BN, NM, TWO, KIND, RING, SLOTS, HALO, WS, &conv_launch_cfg<BN, NM, (TWO != 0), KIND, RING, SLOTS, HALO, (WS != 0)> }
+static const ConvInstance kConvInstances[] = {
+    // halo forms (kind::f16, fp16-plane input): 3x3 (HALO 1) and the stem (HALO 2)
+    DT_CONV_ROW(128, 1, 1, KIND_F16X3, 0, 2, 1, 0), DT_CONV_ROW(64, 3, 1, KIND_F16X3, 0, 2, 1, 1), DT_CONV_ROW(64, 1, 1, KIND_F16X3, 0, 2, 2, 1),
+    DT_CONV_ROW(64, 3, 1, KIND_F16X3, 0, 2, 2, 1), DT_CONV_ROW(64, 3, 0, KIND_F16X3, 0, 2, 1, 0), DT_CONV_ROW(64, 3, 0, KIND_F16X3, 0, 2, 2, 0),
+    // kind::f16, 2-SM MMA
+    DT_CONV_ROW(64, 1, 1, KIND_F16X3, 0, 2, 0, 0), DT_CONV_ROW(64, 3, 1, KIND_F16X3, 0, 2, 0, 0), DT_CONV_ROW(64, 3, 1, KIND_F16X3, 0, 1, 0, 0),
+    DT_CONV_ROW(128, 3, 1, KIND_F16X3, 0, 2, 0, 0), DT_CONV_ROW(128, 3, 1, KIND_F16X3, 0, 1, 0, 0), DT_CONV_ROW(128, 1, 1, KIND_F16X3, 0, 2, 0, 0),
+    DT_CONV_ROW(128, 1, 1, KIND_F16X3, 0, 1, 0, 0),
+    // residual prefetch ring: 2 tiles in flight per epilogue group with two staging slots (3 with one slot); ring 3 + 2 slots (possible with
+    // 32 KB stages) measured 8-11 % slower than ring 2 + 2 slots
+    DT_CONV_ROW(256, 0, 1, KIND_F16X3, 2, 1, 0, 0), DT_CONV_ROW(256, 0, 1, KIND_F16X3, 3, 1, 0, 0), DT_CONV_ROW(256, 0, 1, KIND_F16X3, 2, 2, 0, 0),
+    DT_CONV_ROW(256, 0, 1, KIND_F16X3, 0, 2, 0, 0), DT_CONV_ROW(256, 0, 1, KIND_F16X3, 0, 1, 0, 0), DT_CONV_ROW(256, 1, 1, KIND_F16X3, 0, 2, 0, 0),
+    DT_CONV_ROW(256, 1, 1, KIND_F16X3, 0, 1, 0, 0),
+    // kind::f16, 1-SM MMA + multicast weights
+    DT_CONV_ROW(64, 1, 0, KIND_F16X3, 0, 2, 0, 0), DT_CONV_ROW(64, 3, 0, KIND_F16X3, 0, 2, 0, 0), DT_CONV_ROW(64, 3, 0, KIND_F16X3, 0, 1, 0, 0),
+    DT_CONV_ROW(128, 3, 0, KIND_F16X3, 0, 2, 0, 0), DT_CONV_ROW(128, 3, 0, KIND_F16X3, 0, 1, 0, 0), DT_CONV_ROW(128, 1, 0, KIND_F16X3, 0, 2, 0, 0),
+    DT_CONV_ROW(128, 1, 0, KIND_F16X3, 0, 1, 0, 0), DT_CONV_ROW(256, 0, 0, KIND_F16X3, 0, 1, 0, 0), DT_CONV_ROW(256, 1, 0, KIND_F16X3, 0, 1, 0, 0),
+    // 3xTF32 (one staging slot: the tf32 kind's stages are 64-96 KB)
+    DT_CONV_ROW(64, 3, 1, KIND_TF32X3, 0, 1, 0, 0), DT_CONV_ROW(128, 3, 1, KIND_TF32X3, 0, 1, 0, 0), DT_CONV_ROW(128, 1, 1, KIND_TF32X3, 0, 1, 0, 0),
+    DT_CONV_ROW(256, 0, 1, KIND_TF32X3, 0, 1, 0, 0), DT_CONV_ROW(256, 1, 1, KIND_TF32X3, 0, 1, 0, 0),
+    DT_CONV_ROW(64, 3, 0, KIND_TF32X3, 0, 1, 0, 0), DT_CONV_ROW(128, 3, 0, KIND_TF32X3, 0, 1, 0, 0), DT_CONV_ROW(128, 1, 0, KIND_TF32X3, 0, 1, 0, 0),
+    DT_CONV_ROW(256, 0, 0, KIND_TF32X3, 0, 1, 0, 0), DT_CONV_ROW(256, 1, 0, KIND_TF32X3, 0, 1, 0, 0),
+};
+#undef DT_CONV_ROW
+constexpr int kNumConvInstances = (int)(sizeof(kConvInstances) / sizeof(kConvInstances[0]));
+
+// The row a built layer runs: its fields, with the combinations a kernel does not exist for folded onto the one that runs them
+// (the tf32 kind and the 1-SM 256-wide tiles have one staging slot; ring layers are told apart by ring size and slots).  -1: none.
+inline int conv_instance_of(const ConvLayer& L) {
+    if (!L.valid) return -1;
+    const bool f16 = L.kind == KIND_F16X3, two = L.two_sm;
+    const bool s2 = f16 && L.slots == 2;
+    int nm = L.nmain, ring = 0, slots = s2 ? 2 : 1;
+    if (L.halo) {
+        if (!f16) return -1;
+        if (L.block_n == 64 && L.halo == 1 && !L.ws) nm = 3;
+        if (L.block_n == 64 && L.halo == 2 && !L.ws) nm = 3;
+        if (L.block_n == 64 && L.halo == 2 && L.ws && nm != 1) nm = 3;
+        slots = 2;
+    } else if (L.block_n == 64) {
+        if (!(f16 && nm == 1 && s2)) nm = 3;
+    } else if (L.block_n == 128) {
+        if (nm != 3) nm = 1;
+    } else if (L.block_n == 256) {
+        if (nm == 0 && two && f16 && L.ring) { ring = (s2 || L.ring == 2) ? 2 : 3; }
+        else if (!(two && f16)) slots = 1;
+        if (nm != 0) nm = 1;
     }
-    switch (L.block_n) {
-        case 64:
-            if constexpr (kCan2) { if (L.nmain == 1 && s2) return conv_launch_cfg<64, 1, TWO, KIND, 0, 2>(L, stream); }
-            return s2 ? conv_launch_cfg<64, 3, TWO, KIND, 0, S2>(L, stream) : conv_launch_cfg<64, 3, TWO, KIND, 0, 1>(L, stream);
-        case 128:
-            if (L.nmain == 3) return s2 ? conv_launch_cfg<128, 3, TWO, KIND, 0, S2>(L, stream) : conv_launch_cfg<128, 3, TWO, KIND, 0, 1>(L, stream);
-            return s2 ? conv_launch_cfg<128, 1, TWO, KIND, 0, S2>(L, stream) : conv_launch_cfg<128, 1, TWO, KIND, 0, 1>(L, stream);
-        case 256:
-            if (L.nmain == 0) {
-                if constexpr (TWO && KIND == KIND_F16X3) {
-                    if (L.ring) {
-                        // residual prefetch ring: 2 tiles in flight per epilogue group with two staging slots (3 with one slot);
-                        // ring 3 + 2 slots (possible with 32 KB stages) measured 8-11 % slower than ring 2 + 2 slots
-                        if (!s2) return L.ring == 2 ? conv_launch_cfg<256, 0, TWO, KIND, 2, 1>(L, stream) : conv_launch_cfg<256, 0, TWO, KIND, 3, 1>(L, stream);
-                        return conv_launch_cfg<256, 0, TWO, KIND, 2, 2>(L, stream);
-                    }
-                    if (s2) return conv_launch_cfg<256, 0, TWO, KIND, 0, 2>(L, stream);
-                }
-                return conv_launch_cfg<256, 0, TWO, KIND, 0, 1>(L, stream);
-            }
-            if constexpr (TWO && KIND == KIND_F16X3) { if (s2) return conv_launch_cfg<256, 1, TWO, KIND, 0, 2>(L, stream); }
-            return conv_launch_cfg<256, 1, TWO, KIND>(L, stream);
-        default: return cudaErrorInvalidValue;
+    const int ws = L.ws ? 1 : 0;
+    for (int i = 0; i < kNumConvInstances; ++i) {
+        const ConvInstance& r = kConvInstances[i];
+        if (r.bn == L.block_n && r.nmain == nm && r.two_sm == (two ? 1 : 0) && r.kind == L.kind && r.ring == ring && r.slots == slots &&
+            r.halo == L.halo && r.ws == ws)
+            return i;
     }
+    return -1;
 }
 
 inline cudaError_t conv_launch(const ConvLayer& L, cudaStream_t stream) {
-    if (!L.valid) return cudaErrorInvalidValue;
-    if (L.kind == KIND_F16X3) return L.two_sm ? conv_launch_sm<true, KIND_F16X3>(L, stream) : conv_launch_sm<false, KIND_F16X3>(L, stream);
-    return L.two_sm ? conv_launch_sm<true, KIND_TF32X3>(L, stream) : conv_launch_sm<false, KIND_TF32X3>(L, stream);
+    const int i = conv_instance_of(L);
+    if (i < 0) return cudaErrorInvalidValue;
+    return kConvInstances[i].launch(L, stream);
 }
 
 }  // namespace dt

@@ -98,6 +98,7 @@ struct ConvParams {
     int* range_flag;       // KIND_F16X3: set to 1 when an activation does not fit fp16 (|x| >= 65504 or NaN); may be null
     int pdl;               // launched with programmatic stream serialization: release the next launch early, wait for the previous one
     int a_halo_bytes;      // HALO variant: bytes of ONE fp16 plane of the (wbox + 2) x hbox x nbox halo box (rows of 64 B)
+    float a_mult;          // KIND_F16X3, fp32 input: power of two the converters apply before the fp16 split (0 = none; the engine passes none)
 };
 
 // HALO (3x3, stride 1, fp16-plane input, tiles 8 pixels wide): one TMA box of (8 + 2) x hbox x nbox pixels per (filter row, 32-channel
@@ -507,6 +508,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__((ConvCfg<BLOCK_N, NM
                         float4 fin[8];
 #pragma unroll
                         for (int i = 0; i < 8; ++i) fin[i] = *reinterpret_cast<const float4*>(a32 + r * 128 + ((i ^ (r & 7)) << 4));
+                        if (p.a_mult != 0.f) {
+                            // exact (a power of two): lifts small activations out of the range where the low half is subnormal
+#pragma unroll
+                            for (int i = 0; i < 8; ++i) { fin[i].x *= p.a_mult; fin[i].y *= p.a_mult; fin[i].z *= p.a_mult; fin[i].w *= p.a_mult; }
+                        }
                         named_bar_sync(3, Cfg::CONV_THREADS);          // ids 1, 2 belong to the epilogue groups
 #pragma unroll
                         for (int c8 = 0; c8 < 4; ++c8) {
@@ -542,7 +548,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__((ConvCfg<BLOCK_N, NM
                             const int r = ct & 127, c8 = (ct >> 7) * PIECES + i;
                             const float4 v0 = *reinterpret_cast<const float4*>(a32 + r * 128 + (((2 * c8) ^ (r & 7)) << 4));
                             const float4 v1 = *reinterpret_cast<const float4*>(a32 + r * 128 + (((2 * c8 + 1) ^ (r & 7)) << 4));
-                            const float f[8] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w};
+                            float f[8] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w};
+                            if (p.a_mult != 0.f) {
+#pragma unroll
+                                for (int j = 0; j < 8; ++j) f[j] *= p.a_mult;
+                            }
                             __half2 hh[4], ll[4];
 #pragma unroll
                             for (int j = 0; j < 4; ++j) {

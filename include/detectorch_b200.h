@@ -153,6 +153,51 @@ int dt_conv2d_nhwc(const float* x, int N, int H, int W, int Cin, int x_pix_strid
                    int res_mode, const float* up_src, int up_h, int up_w, int relu, int sigmoid_ch, int passes, int force_block_n,
                    float* y, int y_pix_stride, dt_stream_t stream);
 
+/* Any single conv layer the engine can run, with every option of its layers: fp16 hi/lo plane input (x_lo) and output (y_lo, f16 kind,
+ * dense layout, Cout % 32 == 0), the filter-tap range of a K-split (taps [tap0, tap0 + ntaps), ntaps 0 = all), the scattered output of a
+ * transposed conv (out_step != 0: output pixel (n,h,w) is written at pixel (n, h*out_step + out_y0, w*out_step + out_x0) of an
+ * [N,out_h,out_w] map), channel-slice input / wider output buffers (pixel strides; 0 = dense), the precise / unmerged accumulator forms.
+ * kind 0 = 3xTF32 (w_hi fp32, w_lo = dt_tf32_residual), 1 = the kind::f16 product (w_hi / w_lo from dt_fp16_split).  x_multiplier
+ * (f16 kind, fp32 input; 0 or 1 = none) is a power of two applied to x before the fp16 split: it keeps the low halves of small
+ * activations normal fp16 numbers; the caller folds 1 / x_multiplier into scale like the weight multiplier.
+ * plan_out (host, may be NULL) receives the tile geometry and the kernel instantiation the layer runs; launch 0 only plans. */
+typedef struct dt_conv_desc {
+    int kind;
+    const void* x; const void* x_lo;
+    int N, H, W, Cin, x_pix_stride;
+    float x_multiplier;
+    const void* w_hi; const void* w_lo;
+    int Cout, kh, kw, pad, stride;
+    const float* scale; const float* shift;
+    void* y; void* y_lo; int y_pix_stride;
+    int out_h, out_w, out_step, out_y0, out_x0;
+    const float* residual; int res_pix_stride;
+    const float* up_src; int up_h, up_w;
+    int res_mode, relu, sigmoid_ch, passes;
+    int tap0, ntaps;
+    int force_block_n, precise, no_merge;
+    int* range_flag;
+} dt_conv_desc;
+
+typedef struct dt_conv_plan {
+    int instantiation;                                 /* row of the instantiation table below (-1: none) */
+    int block_n, nmain, two_sm, kind, ring, slots, halo, ws;   /* that row; nmain 0 = one merged accumulator, 1, or 3 rotating */
+    int wbox, hbox, nbox, tiles_w, tiles_h, tiles_n;   /* output tile box and tile counts */
+    int m_pairs, n_tiles, grid;                        /* work items = m_pairs * n_tiles over `grid` CTAs (2 per cluster) */
+    int num_kb;                                        /* 32-element k-blocks per tile */
+    int ho, wo;
+} dt_conv_plan;
+
+int dt_conv2d_spec(const dt_conv_desc* desc, dt_conv_plan* plan_out, int launch, dt_stream_t stream);
+/* The 7x7 stride-2 stem (3 input channels) over a zero-bordered NHWC4 image x4 [B,Hp,Wp,4] (3-pixel border, channel 3 = 0,
+ * Hp >= 2*H1 + 5, Wp >= 2*W1 + 6), or (planes != 0, f16 kind, Wp even) its fp16 hi and lo planes back to back; weights [64][7 (ky)][32]
+ * (element kx*4 + c, zero for kx = 7 or c = 3); y [B,H1,W1,64], ReLU applied. */
+int dt_conv2d_stem(const void* x4, int planes, int B, int Hp, int Wp, int H1, int W1, const void* w_hi, const void* w_lo, int kind,
+                   const float* scale, const float* shift, float x_multiplier, int passes, int* range_flag, float* y, dt_conv_plan* plan_out,
+                   int launch, dt_stream_t stream);
+/* the kernel instantiation table: fields8 = {block_n, nmain, two_sm, kind, ring, slots, halo, ws} of row i */
+int dt_conv_instantiation_count(void);
+int dt_conv_instantiation_info(int i, int* fields8);
 
 /* ---------------------------------------------------------------------------------------------
  * Fused Mask R-CNN (ResNet-50/101 + FPN) inference engine: the whole of

@@ -1,6 +1,6 @@
 """GPU bring-up probe (not a pytest file): runs groups of operator checks against the oracle and
 prints one line per case.  Used under gpurun with a per-group `timeout` so a hung kernel cannot
-hang the box:   timeout 300 python tests/gpu_probe.py conv_basic
+hang the box:   timeout 300 python tests/gpu_probe.py roialign nms
 """
 import os
 import sys
@@ -14,84 +14,6 @@ from detectorch_b200 import ops  # noqa: E402
 from oracle import ref  # noqa: E402
 
 dev = torch.device("cuda:0")
-
-
-def conv_ref(x_nhwc, w, scale, shift, kh, kw, pad, stride, residual=None, up=None, relu=False, sigmoid_ch=0):
-    """fp64 reference on CPU. w: [Cout, kh, kw, Cin]."""
-    x = x_nhwc.double().permute(0, 3, 1, 2)
-    wt = w.double().permute(0, 3, 1, 2)
-    y = torch.nn.functional.conv2d(x, wt, stride=stride, padding=pad)
-    y = y * scale.double().view(1, -1, 1, 1) + shift.double().view(1, -1, 1, 1)
-    if residual is not None:
-        y = y + residual.double().permute(0, 3, 1, 2)
-    if up is not None:
-        u = torch.nn.functional.interpolate(up.double().permute(0, 3, 1, 2), scale_factor=2, mode="nearest")
-        y = y + u[:, :, :y.size(2), :y.size(3)]
-    if relu:
-        y = torch.relu(y)
-    y = y.permute(0, 2, 3, 1).contiguous()
-    if sigmoid_ch:
-        y[..., :sigmoid_ch] = torch.sigmoid(y[..., :sigmoid_ch])
-    return y
-
-
-def run_conv(tag, N, H, W, Cin, Cout, kh, pad, stride, passes=3, res=False, up=False, relu=False, sigmoid_ch=0, bn=0, seed=0):
-    g = torch.Generator().manual_seed(seed)
-    x = torch.randn((N, H, W, Cin), generator=g)
-    w = torch.randn((Cout, kh, kh, Cin), generator=g) * (2.0 / (kh * kh * Cin)) ** 0.5
-    scale = 0.5 + torch.rand((Cout,), generator=g)
-    shift = 0.1 * torch.randn((Cout,), generator=g)
-    Ho = (H + 2 * pad - kh) // stride + 1
-    Wo = (W + 2 * pad - kh) // stride + 1
-    residual = torch.randn((N, Ho, Wo, Cout), generator=g) if res else None
-    upsrc = torch.randn((N, (Ho + 1) // 2, (Wo + 1) // 2, Cout), generator=g) if up else None
-    want = conv_ref(x, w, scale, shift, kh, kh, pad, stride, residual, upsrc, relu, sigmoid_ch)
-    t0 = time.time()
-    got = ops.conv2d_nhwc(x.to(dev), w.reshape(Cout, -1).contiguous().to(dev), scale.to(dev), shift.to(dev), kh, kh, pad, stride,
-                          residual=residual.to(dev) if res else None, up_src=upsrc.to(dev) if up else None, relu=relu,
-                          sigmoid_ch=sigmoid_ch, passes=passes, force_block_n=bn)
-    torch.cuda.synchronize()
-    got = got.cpu().double()
-    err = (got - want).abs()
-    denom = want.abs().max().item()
-    bad = int((err > 1e-3 * max(denom, 1.0)).sum())
-    print("CONV %-28s N%d %dx%d Cin%d Cout%d k%d s%d p%d bn%d passes%d : max_abs_err %.3e (ref max %.3f) rel %.3e bad %d/%d  %.2fs" % (
-        tag, N, H, W, Cin, Cout, kh, stride, pad, bn, passes, err.max().item(), denom, err.max().item() / max(denom, 1e-9), bad,
-        err.numel(), time.time() - t0), flush=True)
-    if bad and err.numel() < 10**7:
-        idx = torch.nonzero(err > 1e-3 * max(denom, 1.0))
-        print("   first bad idx:", idx[:6].tolist(), "got", [got[tuple(i)].item() for i in idx[:3]], "want",
-              [want[tuple(i)].item() for i in idx[:3]], flush=True)
-        rows = torch.unique(idx[:, 1] * 100000 + idx[:, 2])
-        chans = torch.unique(idx[:, 3])
-        print("   bad pixels %d  bad channels %d (first %s)" % (len(rows), len(chans), chans[:16].tolist()), flush=True)
-    return err.max().item() / max(denom, 1e-9)
-
-
-def group_conv_basic():
-    run_conv("gemm64 1pass", 1, 1, 128, 64, 64, 1, 0, 1, passes=1)
-    run_conv("gemm64 3pass", 1, 1, 128, 64, 64, 1, 0, 1, passes=3)
-    run_conv("gemm K256 bn128", 1, 1, 384, 256, 128, 1, 0, 1, passes=3)
-    run_conv("gemm K256 bn256", 1, 1, 384, 256, 256, 1, 0, 1, passes=3)
-    run_conv("gemm K1024 N512", 1, 1, 1000, 1024, 512, 1, 0, 1, passes=3)
-
-
-def group_conv_spatial():
-    run_conv("1x1 16x24", 1, 16, 24, 64, 64, 1, 0, 1)
-    run_conv("3x3 20x30", 1, 20, 30, 64, 128, 3, 1, 1)
-    run_conv("3x3 25x38 N2", 2, 25, 38, 256, 256, 3, 1, 1)
-    run_conv("1x1 s2", 1, 50, 76, 256, 128, 1, 0, 2)
-    run_conv("1x1 s2 odd", 2, 25, 38, 128, 64, 1, 0, 2)
-    run_conv("mask 14x14 N5", 5, 14, 14, 256, 256, 3, 1, 1)
-
-
-def group_conv_epilogue():
-    run_conv("res+relu", 1, 20, 30, 64, 256, 1, 0, 1, res=True, relu=True)
-    run_conv("res+relu bn64", 2, 13, 19, 128, 64, 3, 1, 1, res=True, relu=True)
-    run_conv("upsample", 1, 26, 38, 64, 256, 1, 0, 1, up=True)
-    run_conv("rpn head 16ch sigmoid", 1, 25, 38, 256, 16, 1, 0, 1, sigmoid_ch=3)
-    run_conv("cout 408", 1, 1, 1000, 1024, 408, 1, 0, 1)
-    run_conv("big 200x304 3x3", 1, 200, 304, 64, 64, 3, 1, 1, relu=True)
 
 
 def group_roialign():

@@ -332,24 +332,6 @@ def test_conv_f16_epilogues_tiles_and_range_flag(dev):
     assert int(flag.item()) == 1
 
 
-def test_conv_both_mma_modes(built):
-    """The 1-SM (multicast) and 2-SM (cta_group::2) variants of the conv kernel are both exercised over every tile
-    configuration in fresh processes (the mode is latched per process from DT_CONV_MMA)."""
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    for mode in ("1sm", "2sm"):
-        env = dict(os.environ, DT_CONV_MMA=mode)
-        out = subprocess.run([sys.executable, os.path.join(root, "tests", "gpu_probe.py"), "conv_basic", "conv_spatial", "conv_epilogue"],
-                             env=env, capture_output=True, text=True, timeout=600)
-        assert out.returncode == 0, out.stderr[-2000:]
-        lines = [l for l in out.stdout.splitlines() if l.startswith("CONV")]
-        assert len(lines) == 17
-        for l in lines:
-            rel = float(l.split(" rel ")[1].split()[0])
-            assert rel < (5e-3 if "passes1" in l else 1e-4), (mode, l)
-
-
 def test_conv_epilogues(dev):
     assert _conv_case(dev, 1, 20, 30, 64, 256, 1, 0, 1, res=True, relu=True) < 1e-4
     assert _conv_case(dev, 2, 13, 19, 128, 64, 3, 1, 1, res=True, relu=True) < 1e-4

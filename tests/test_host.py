@@ -32,8 +32,33 @@ def test_library_exports_every_declared_symbol(built):
 def test_ctypes_signatures_cover_operator_api(built):
     from detectorch_b200 import _lib
     for n in ("launch_roi_align_forward_cuda", "launch_roi_align_backward_cuda", "dt_roi_align_forward_nchw", "dt_roi_align_forward_nhwc", "dt_nms",
-              "dt_conv2d_nhwc", "dt_conv2d_nhwc_f16x3", "dt_fp16_split", "dt_segm_rle", "dt_segm_paste", "dt_prep_image"):
+              "dt_conv2d_nhwc", "dt_conv2d_nhwc_f16x3", "dt_conv2d_spec", "dt_conv2d_stem", "dt_conv_instantiation_count",
+              "dt_conv_instantiation_info", "dt_fp16_split", "dt_segm_rle", "dt_segm_paste", "dt_prep_image"):
         assert n in _lib.SIGNATURES
+
+
+def test_conv_desc_and_plan_structs_match_header(built):
+    """The ctypes mirrors of dt_conv_desc / dt_conv_plan list the header's fields in the header's order with the same C types, and the
+    instantiation table is exported (39 rows of distinct kernel template arguments)."""
+    from detectorch_b200 import _lib
+    src = re.sub(r"/\*.*?\*/", "", open(os.path.join(ROOT, "include", "detectorch_b200.h")).read(), flags=re.S)
+    ctype = {"int": ctypes.c_int, "float": ctypes.c_float}
+    for cname, py in (("dt_conv_desc", _lib.ConvDesc), ("dt_conv_plan", _lib.ConvPlan)):
+        body = re.search(r"typedef struct %s \{(.*?)\} %s;" % (cname, cname), src, re.S).group(1)
+        fields = []
+        for decl in body.split(";"):
+            decl = " ".join(decl.split())
+            if not decl:
+                continue
+            m = re.match(r"(const )?(int|float|void|char)\s*(\*?)\s*(.*)", decl)
+            base, ptr = m.group(2), m.group(3)
+            for name in m.group(4).split(","):
+                name = name.strip()
+                star = ptr or name.startswith("*")
+                fields.append((name.lstrip("* "), ctypes.c_void_p if star else ctype[base]))
+        assert [(f, t) for f, t in py._fields_] == fields, cname
+    rows = __import__("detectorch_b200.ops", fromlist=["ops"]).conv_instantiations()
+    assert len(rows) == 39 and len(set(rows)) == 39
 
 
 def test_engine_param_table_matches_reference_names(built):
